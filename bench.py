@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — cells / second / Harmony-iteration on synthetic embeddings (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -16,6 +16,9 @@ ranks), `e2e` (the same metric through the public API with HOST buffers: setup H
 getZcorr D2H), `roofline` (dominant kernel, algorithmic bytes / measured launch time, against
 MEASURED_PEAKS.json) and `cpu_baseline` (the CPU oracle = restatement of the reference, timed on this
 box's host cores on a bounded sample).
+
+`--dump-outputs DIR` writes what the timed path handed its caller after the last timed step (see dump_outputs), so
+that two builds run with the same arguments, and therefore the same inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -290,6 +293,26 @@ def parity_on_sample(device, n_cells=50_000, iters=2, seed=20260926):
     return out
 
 
+DUMP_CELLS = 32_768     # 39 MB of float32 at the widest workload (c5: d=100, K=200)
+
+
+def dump_outputs(g, n_local, out_dir, seed=20261017):
+    """Writes DIR/<name>.npy: the corrected embedding (getZcorr, d x cells) and the soft cluster assignments
+    (R, K x cells) of a fixed, seeded sample of DUMP_CELLS cells of this rank's shard, in shard order, the
+    centroids (Y, d x K) and the last Harmony objective.  The library holds its state in fp32, so Z_corr, R and Y
+    are stored as float32 without loss; the objective stays float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    cells = np.sort(np.random.default_rng(seed).choice(n_local, min(n_local, DUMP_CELLS), replace=False))
+    out = {"Z_corr": g.getZcorr()[:, cells].astype(np.float32),      # one full download at a time
+           "R": g.getR()[:, cells].astype(np.float32),
+           "Y": g.getCentroids().astype(np.float32),
+           "objective_harmony": g.objective_harmony[-1:].astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+    log(f"outputs of the last timed step written to {out_dir}: "
+        + ", ".join(f"{k} {v.shape} {v.dtype}" for k, v in out.items()))
+
+
 def run_reference(args):
     """--impl reference: the reference's own CPU algorithm (oracle port) with all host BLAS threads."""
     rank = int(os.environ.get("RANK", "0"))
@@ -297,7 +320,7 @@ def run_reference(args):
         return
     ncpu = os.cpu_count() or 1
     n_sample = int(args.ref_cells) if args.ref_cells > 0 else cpu_sample_cells()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     # the reference only threads its BLAS call (R/ui.R:123-128); time it with all host threads and with the
     # reference default ncores = 1 and report the faster of the two (skinny sgemm often loses with threads)
     t_all, blas = cpu_reference_run(n_sample, steps, ncpu)
@@ -331,7 +354,13 @@ def main():
     ap.add_argument("--clock-period", type=float, default=0.003, help="seconds between NVML clock samples during the timed region")
     ap.add_argument("--kernel-set", type=int, default=0, help="HB_KERNEL_SET test hook of the library (A/B runs only)")
     ap.add_argument("--ref-cells", type=int, default=0, help="cells of the bounded CPU sample (--impl reference); 0 = by workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (rank 0's shard; --impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     W.clear()
     W.update(WORKLOADS[args.config])
     if args.cells_per_gpu <= 0:
@@ -443,6 +472,8 @@ def main():
         dist.all_reduce(tm, op=dist.ReduceOp.MAX)
         ms = float(tm.item())
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(g, n_local, args.dump_outputs)
     ms_per_step = ms / args.steps
     value = N_global / (ms_per_step * 1e-3)
 
