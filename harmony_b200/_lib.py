@@ -12,7 +12,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
 SO_PATH = os.path.join(_HERE, "libharmony_b200.so")
 SOURCES = [os.path.join(_HERE, "csrc", f) for f in ("harmony_b200.cu", "kernels.cuh", "common.cuh", "update_kernel.cuh", "update_kernel4.cuh", "update_kernel5.cuh",
-                                                     "umma.cuh", "assign_tc3.cuh", "logits_tc.cuh", "stats_tc3.cuh", "apply_tc3.cuh")]
+                                                     "umma.cuh", "assign_tc3.cuh", "logits_tc.cuh", "stats_tc3.cuh", "apply_tc3.cuh",
+                                                     "setup_device.cuh")]
 HEADER = os.path.join(ROOT, "include", "harmony_b200.h")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC"]
@@ -67,6 +68,7 @@ def lib():
     L.hb_comm_init.argtypes = [P, I, I, ctypes.c_char_p]
     L.hb_set_shard.argtypes = [P, I64, I64]
     L.hb_setup.argtypes = [P, P, I, I64, P, P, I, P, P, P, D, I, D, D, I, D, D, I]
+    L.hb_setup_device.argtypes = [P, P, I, I64, I64, I, I64, P, P, I, P, P, P, D, I, D, D, I, D, D, I, P]
     L.hb_set_seed.argtypes = [P, ctypes.c_uint64]
     L.hb_set_abort_callback.argtypes = [P, P, P]
     L.hb_init_cluster.argtypes = [P, P]
@@ -78,6 +80,7 @@ def lib():
     L.hb_field_size.argtypes = [P, I]
     L.hb_get_field.argtypes = [P, I, P]
     L.hb_set_field.argtypes = [P, I, P]
+    L.hb_get_field_device.argtypes = [P, I, P, I, I64, P]
     L.hb_get_scalar.argtypes = [P, I, ctypes.POINTER(D)]
     L.hb_set_scalar.argtypes = [P, I, D]
     L.hb_get_B_vec.argtypes = [P, P]
@@ -96,6 +99,7 @@ def lib():
     L.hb_debug_kmeans_uniform.restype = D
     L.hb_debug_kmeans_uniform.argtypes = [P, ctypes.c_uint64, ctypes.c_uint64]
     L.hb_debug_kmeans_cells.argtypes = [P, P]
+    L.hb_debug_sort_perm.argtypes = [P, P]
     L.hb_debug_widen.argtypes = [P, P, I64, I]
     _LIB = L
     return L

@@ -34,6 +34,7 @@
 #include "logits_tc.cuh"
 #include "apply_tc3.cuh"
 #include "stats_tc3.cuh"
+#include "setup_device.cuh"
 
 namespace {
 
@@ -333,7 +334,6 @@ struct hb_handle {
   int ntiles = 0, nchunks = 0;  // nchunks includes the trailing empty chunk
   int trace_cap = 0;
   std::vector<int> tuple_levels_h;  // [J][C]
-  std::vector<int> sort_perm_h;
   std::vector<int64_t> kmeans_cells;  // global cells chosen by the native initialize_centroids (test hook)
 
   // traces (harmony.h:55-56); values are produced on the device and pulled lazily
@@ -352,6 +352,7 @@ struct hb_handle {
   bool timing = false;
   std::map<std::string, Region> regions;
   cudaEvent_t ev0 = nullptr;  // orders the side-stream plan build after the main stream
+  cudaEvent_t io_ev = nullptr;  // orders device-memory inputs / outputs against the caller's stream
 };
 
 namespace {
@@ -1496,8 +1497,8 @@ int download_rows_mt(hb_handle* h, const float* src, int cols, int ld, double* o
   auto enqueue = [&](int64_t i) -> int {
     const int64_t r0 = i * rows_per, rows = std::min(rows_per, n - r0);
     float* d = dev + (size_t)(i & 1) * dev_half;
-    k_download_rows_f<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(src, d, h->inv_sort.p, r0, rows,
-                                                                                         cols, ld);
+    k_download_rows<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(src, d, (int64_t)cols, h->inv_sort.p,
+                                                                                       r0, rows, cols, ld);
     CKL();
     CK(cudaMemcpyAsync(pinned[i & 1], d, sizeof(float) * (size_t)rows * cols, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaEventRecord(ev[i & 1], h->stream));
@@ -1530,8 +1531,8 @@ int download_rows(hb_handle* h, const float* src, int cols, int ld, double* out)
   const int64_t rows_per = std::max<int64_t>(1, (int64_t)(h->stage.n / (size_t)cols));
   for (int64_t r0 = 0; r0 < n; r0 += rows_per) {
     int64_t rows = std::min(rows_per, n - r0);
-    k_download_rows<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(src, h->stage.p, h->inv_sort.p,
-                                                                                        r0, rows, cols, ld);
+    k_download_rows<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(src, h->stage.p, (int64_t)cols,
+                                                                                        h->inv_sort.p, r0, rows, cols, ld);
     CKL();
     CK(cudaMemcpyAsync(out + r0 * cols, h->stage.p, sizeof(double) * (size_t)rows * cols, cudaMemcpyDeviceToHost,
                        h->stream));
@@ -1546,8 +1547,8 @@ int upload_rows(hb_handle* h, const double* in, int cols, int ld, float* dst) {
     int64_t rows = std::min(rows_per, n - r0);
     CK(cudaMemcpyAsync(h->stage.p, in + r0 * cols, sizeof(double) * (size_t)rows * cols, cudaMemcpyHostToDevice,
                        h->stream));
-    k_upload_rows<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->stage.p, dst, h->inv_sort.p, r0,
-                                                                                      rows, cols, ld);
+    k_upload_rows<<<grid_for(rows * cols, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->stage.p, (int64_t)cols, (int64_t)1,
+                                                                                      dst, h->inv_sort.p, r0, rows, cols, ld);
     CKL();
     CK(cudaStreamSynchronize(h->stream));
   }
@@ -1588,6 +1589,552 @@ int upload_small(hb_handle* h, const double* in, size_t count, float* dst) {
   return 0;
 }
 
+// ---- pieces of hb_setup / hb_setup_device, in the order they run ------------------------------------
+// (a) arguments and scalars (harmony.cpp:29-91)
+int setup_scalars(hb_handle* h, const void* Z, int d, int64_t N, const void* phi_i, const int32_t* B_vec, int C,
+                  const double* sigma, const double* theta, const double* lambda, double alpha, int max_iter_kmeans,
+                  double epsilon_kmeans, double epsilon_harmony, int K, double block_size,
+                  double batch_proportion_cutoff, int verbose) {
+  if (h->ran_setup) return fail(h, 3, "setup was already run on this object");
+  if (!Z || !phi_i || !B_vec || !sigma || !theta) return fail(h, 2, "null argument");
+  if (d < 1 || N < 1 || C < 1 || K < 1) return fail(h, 2, "bad dimensions");
+  if (K > 1024) return fail(h, 2, "K = %d is not supported (K <= 1024)", K);
+  if (N > 2000000000LL) return fail(h, 2, "more than 2e9 cells per GPU are not supported");
+  CK(cudaSetDevice(h->device));
+  h->n = N;
+  if (!h->shard_set) {
+    if (h->world > 1) return fail(h, 3, "hb_set_shard is required when world_size > 1");
+    h->N_global = N;
+    h->cell_offset = 0;
+  }
+  const int64_t NG = h->N_global;
+  h->d = d;
+  h->C = C;
+  h->K = K;
+  h->KS = (K + 3) & ~3;
+  h->DS = (d + 3) & ~3;
+  h->B_vec.assign(B_vec, B_vec + C);
+  h->B = std::accumulate(h->B_vec.begin(), h->B_vec.end(), 0);
+  const int B = h->B;
+  h->cov_of.resize(B);
+  {
+    int b = 0;
+    for (int c = 0; c < C; ++c)
+      for (int l = 0; l < B_vec[c]; ++l) h->cov_of[b++] = c;
+  }
+  // harmony.cpp:83-91
+  if (NG < 6) return fail(h, 1, "Refusing to run with less than 6 cells");
+  if (NG < 40) {
+    h->warnings.push_back("Too few cells. Setting block_size to 0.2");
+    h->block_size = 0.2f;
+  } else {
+    h->block_size = (float)block_size;
+  }
+  h->epsilon_kmeans = (float)epsilon_kmeans;
+  h->epsilon_harmony = (float)epsilon_harmony;
+  h->alpha = (float)alpha;
+  h->cutoff = (float)batch_proportion_cutoff;
+  h->max_iter_kmeans = (unsigned)max_iter_kmeans;
+  h->verbose = verbose;
+  h->lambda_estimation = (lambda == nullptr) || (lambda[0] == -1);  // harmony.cpp:75
+  // update_R block geometry, harmony.cpp:280-281 (float arithmetic on the GLOBAL cell count)
+  h->nb = my_ceil(1.0f / h->block_size);
+  h->cpb = (uint32_t)((float)NG * h->block_size);
+  if (h->cpb == 0) return fail(h, 2, "block_size * N < 1");
+  {
+    int bits = 1;
+    while ((1ull << bits) < (uint64_t)NG) bits++;
+    h->half_bits = (bits + 1) / 2;
+  }
+  return 0;
+}
+
+constexpr uint64_t kSmallKeySpace = 1ull << 22;  // the usual case: a direct table beats sorting N keys
+
+// Radices of the joint covariate key (the last covariate varies fastest) and the size of the key space.
+int tuple_radix(hb_handle* h, std::vector<uint64_t>& radix, uint64_t* key_space) {
+  const int C = h->C;
+  long double prod = 1;
+  for (int c = 0; c < C; ++c) prod *= (long double)h->B_vec[c];
+  if (prod > 9e18L) return fail(h, 2, "covariate level product overflows 64 bits");
+  radix.assign(C, 0);
+  uint64_t r = 1;
+  for (int c = C - 1; c >= 0; --c) {
+    radix[c] = r;
+    r *= (uint64_t)h->B_vec[c];
+  }
+  *key_space = r;
+  return 0;
+}
+
+// h->J and h->tuple_levels_h from the ascending unique keys
+int set_tuples(hb_handle* h, const std::vector<uint64_t>& uniq, const std::vector<uint64_t>& radix) {
+  if (uniq.size() > 1000000) return fail(h, 2, "more than 1e6 distinct covariate tuples are not supported");
+  const int J = (int)uniq.size(), C = h->C;
+  h->J = J;
+  h->tuple_levels_h.resize((size_t)J * C);
+  std::vector<int> base(C, 0);
+  for (int c = 1; c < C; ++c) base[c] = base[c - 1] + h->B_vec[c - 1];
+  for (int q = 0; q < J; ++q) {
+    uint64_t kk = uniq[q];
+    for (int c = 0; c < C; ++c) {
+      h->tuple_levels_h[(size_t)q * C + c] = base[c] + (int)(kk / radix[c]);
+      kk %= radix[c];
+    }
+  }
+  return 0;
+}
+
+// (b) on the host: joint covariate tuples, level counts (summed over ranks) and the stable sort of the cells by tuple.
+// Sets h->J / h->tuple_levels_h, fills the device sort_perm / inv_sort and returns the first position of every tuple
+// (tstart, J + 1 values).
+int tuple_dict_host(hb_handle* h, const int32_t* phi_i, std::vector<int64_t>& lvl_count, std::vector<int64_t>& tstart) {
+  const int64_t N = h->n;
+  const int C = h->C, B = h->B;
+  const int* B_vec = h->B_vec.data();
+  lvl_count.assign(B, 0);
+  std::vector<uint64_t> key(N);
+  std::vector<uint64_t> radix;
+  uint64_t key_space = 1;
+  TRY(tuple_radix(h, radix, &key_space));
+  {
+    std::vector<int> base(C, 0);
+    for (int c = 1; c < C; ++c) base[c] = base[c - 1] + B_vec[c - 1];
+    for (int64_t i = 0; i < N; ++i) {
+      uint64_t kk = 0;
+      for (int c = 0; c < C; ++c) {
+        int b = phi_i[i * C + c];
+        if (b < base[c] || b >= base[c] + B_vec[c]) return fail(h, 2, "phi row index %d of cell %lld is not a level of covariate %d", b, (long long)i, c);
+        lvl_count[b]++;
+        kk += (uint64_t)(b - base[c]) * radix[c];
+      }
+      key[i] = kk;
+    }
+  }
+  std::vector<uint64_t> uniq;
+  const bool small_space = key_space <= kSmallKeySpace;
+  if (small_space) {
+    std::vector<uint8_t> seen((size_t)key_space, 0);
+    for (int64_t i = 0; i < N; ++i) seen[key[i]] = 1;
+    for (uint64_t k2 = 0; k2 < key_space; ++k2)
+      if (seen[k2]) uniq.push_back(k2);
+  } else {
+    uniq = key;
+    std::sort(uniq.begin(), uniq.end());
+    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
+  }
+  if (h->world > 1) {
+    // global tuple dictionary = union over ranks; level counts summed over ranks
+    long long cnt = (long long)uniq.size(), maxcnt = 0;
+    DevBuf<long long> dcnt;
+    CK(dcnt.alloc(1));
+    CK(cudaMemcpyAsync(dcnt.p, &cnt, sizeof(cnt), cudaMemcpyHostToDevice, h->stream));
+    CKN(g_nccl.AllReduce(dcnt.p, dcnt.p, 1, ncclInt64, ncclMax, h->comm, h->stream));
+    CK(cudaMemcpyAsync(&maxcnt, dcnt.p, sizeof(cnt), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    std::vector<uint64_t> sendbuf((size_t)maxcnt, ~0ull), recvbuf((size_t)maxcnt * h->world);
+    std::copy(uniq.begin(), uniq.end(), sendbuf.begin());
+    DevBuf<uint64_t> ds, dr;
+    CK(ds.alloc((size_t)maxcnt));
+    CK(dr.alloc((size_t)maxcnt * h->world));
+    CK(cudaMemcpyAsync(ds.p, sendbuf.data(), sizeof(uint64_t) * (size_t)maxcnt, cudaMemcpyHostToDevice, h->stream));
+    CKN(g_nccl.AllGather(ds.p, dr.p, (size_t)maxcnt, ncclUint64, h->comm, h->stream));
+    CK(cudaMemcpyAsync(recvbuf.data(), dr.p, sizeof(uint64_t) * recvbuf.size(), cudaMemcpyDeviceToHost, h->stream));
+    DevBuf<long long> dl;
+    CK(dl.alloc(B));
+    std::vector<long long> lc(lvl_count.begin(), lvl_count.end());
+    CK(cudaMemcpyAsync(dl.p, lc.data(), sizeof(long long) * B, cudaMemcpyHostToDevice, h->stream));
+    CKN(g_nccl.AllReduce(dl.p, dl.p, B, ncclInt64, ncclSum, h->comm, h->stream));
+    CK(cudaMemcpyAsync(lc.data(), dl.p, sizeof(long long) * B, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int b = 0; b < B; ++b) lvl_count[b] = lc[b];
+    uniq.assign(recvbuf.begin(), recvbuf.end());
+    std::sort(uniq.begin(), uniq.end());
+    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
+    if (!uniq.empty() && uniq.back() == ~0ull) uniq.pop_back();
+  }
+  TRY(set_tuples(h, uniq, radix));
+  const int J = h->J;
+  std::vector<int> tuple_of(N);
+  tstart.assign(J + 1, 0);
+  {
+    std::vector<int> lut;
+    if (small_space) {
+      lut.assign((size_t)key_space, -1);
+      for (int q = 0; q < J; ++q) lut[uniq[q]] = q;
+    }
+    for (int64_t i = 0; i < N; ++i) {
+      int q = small_space ? lut[key[i]] : (int)(std::lower_bound(uniq.begin(), uniq.end(), key[i]) - uniq.begin());
+      tuple_of[i] = q;
+      tstart[q + 1]++;
+    }
+  }
+  for (int q = 0; q < J; ++q) tstart[q + 1] += tstart[q];
+  std::vector<int> sort_perm(N), inv_sort(N);
+  {
+    std::vector<int64_t> cur(tstart.begin(), tstart.end() - 1);
+    for (int64_t i = 0; i < N; ++i) {
+      int64_t s = cur[tuple_of[i]]++;
+      sort_perm[s] = (int)i;
+      inv_sort[i] = (int)s;
+    }
+  }
+  CK(h->sort_perm.alloc(N));
+  CK(h->inv_sort.alloc(N));
+  CK(cudaMemcpyAsync(h->sort_perm.p, sort_perm.data(), sizeof(int) * N, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(h->inv_sort.p, inv_sort.data(), sizeof(int) * N, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
+// (b) on the device: phi_i is device memory of the handle's device, ordered on h->stream.  Same results as
+// tuple_dict_host (setup_device.cuh); the only host traffic is J + 1 tuple starts and the J unique keys.  A key space
+// above kSmallKeySpace, or more tuples than the counting sort's per-warp shared-memory counters hold, downloads phi_i
+// and runs tuple_dict_host: one implementation serves those rare shapes.
+int tuple_dict_device(hb_handle* h, const int32_t* phi_i, std::vector<int64_t>& lvl_count, std::vector<int64_t>& tstart) {
+  const int64_t N = h->n;
+  const int C = h->C, B = h->B;
+  std::vector<uint64_t> radix;
+  uint64_t key_space = 1;
+  TRY(tuple_radix(h, radix, &key_space));
+  auto on_host = [&]() -> int {
+    std::vector<int32_t> phi((size_t)N * C);
+    CK(cudaMemcpyAsync(phi.data(), phi_i, sizeof(int32_t) * phi.size(), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return tuple_dict_host(h, phi.data(), lvl_count, tstart);
+  };
+  if (key_space > kSmallKeySpace) return on_host();
+  const int KSP = (int)key_space;
+  std::vector<int> lv_h(3 * (size_t)C);
+  for (int c = 0, base = 0; c < C; base += h->B_vec[c], ++c) {
+    lv_h[3 * c] = base;
+    lv_h[3 * c + 1] = h->B_vec[c];
+    lv_h[3 * c + 2] = (int)radix[c];
+  }
+  // ids: presence of every key, then (exclusive scan) its tuple id; int rather than a byte per key because the scan
+  // kernels work on ints.  The trailing word becomes J.
+  DevBuf<int> lv, key, ids;
+  DevBuf<unsigned long long> bad;
+  CK(lv.alloc(lv_h.size()));
+  CK(key.alloc(N));
+  CK(ids.alloc((size_t)KSP + 1));
+  CK(bad.alloc(1));
+  CK(cudaMemcpyAsync(lv.p, lv_h.data(), sizeof(int) * lv_h.size(), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemsetAsync(ids.p, 0, sizeof(int) * ((size_t)KSP + 1), h->stream));
+  CK(cudaMemsetAsync(bad.p, 0xff, sizeof(unsigned long long), h->stream));
+  k_dict_keys<<<grid_for(N, 256, h->num_sms * 8), 256, 0, h->stream>>>(phi_i, N, C, lv.p, key.p, ids.p, bad.p);
+  CKL();
+  unsigned long long first_bad = 0;
+  CK(cudaMemcpyAsync(&first_bad, bad.p, sizeof(first_bad), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  if (first_bad != ~0ull) {  // the host path's report of the same cell
+    int b = 0;
+    CK(cudaMemcpy(&b, phi_i + first_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    return fail(h, 2, "phi row index %d of cell %lld is not a level of covariate %d", b, (long long)(first_bad / C),
+                (int)(first_bad % C));
+  }
+  // global tuple dictionary = union over ranks
+  if (h->world > 1) CKN(g_nccl.AllReduce(ids.p, ids.p, (size_t)KSP, ncclInt32, ncclMax, h->comm, h->stream));
+  DevBuf<unsigned long long> scan_state;
+  auto scan = [&](int* data, int64_t n) -> int {
+    const int tiles = (int)((n + SCAN_TILE - 1) / SCAN_TILE);
+    CK(scan_state.alloc((size_t)tiles + 1));
+    CK(cudaMemsetAsync(scan_state.p, 0, sizeof(unsigned long long) * ((size_t)tiles + 1), h->stream));
+    k_scan_chained<<<dim3(tiles, 1), 1024, 0, h->stream>>>(data, n, scan_state.p, tiles);
+    CKL();
+    return 0;
+  };
+  TRY(scan(ids.p, (int64_t)KSP + 1));
+  int J = 0;
+  CK(cudaMemcpyAsync(&J, ids.p + KSP, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  // stable counting sort by tuple id: one warp per chunk of consecutive cells, J counters per warp in shared memory
+  const size_t per_warp = sizeof(int) * (size_t)J, smem_max = (size_t)227 * 1024 - 256;
+  if (J > 1000000 || per_warp > smem_max) return on_host();
+  const int wpb = (int)std::max<size_t>(1, std::min<size_t>(8, (48 * 1024) / per_warp));
+  const size_t sm = per_warp * wpb;
+  if (sm > 48 * 1024) {
+    CK(cudaFuncSetAttribute(k_plan_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    CK(cudaFuncSetAttribute(k_plan_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  }
+  int CH = 1024;  // histogram of at most 2^24 counters (64 MB)
+  while (CH < N && ((N + CH - 1) / CH) * (int64_t)J > (1 << 24)) CH <<= 1;
+  const int nc = (int)((N + CH - 1) / CH);
+  DevBuf<int> uniq_d, cstart, cq0, cnq, H, tst, flag;
+  CK(uniq_d.alloc(J));
+  CK(cstart.alloc((size_t)nc + 1));
+  CK(cq0.alloc(nc));
+  CK(cnq.alloc(nc));
+  CK(H.alloc((size_t)J * nc));
+  CK(tst.alloc((size_t)J + 1));
+  CK(flag.alloc(1));
+  CK(h->sort_perm.alloc(N));
+  CK(h->inv_sort.alloc(N));
+  k_dict_tuples<<<grid_for(std::max<int64_t>(KSP, N), 256, h->num_sms * 8), 256, 0, h->stream>>>(ids.p, KSP, uniq_d.p,
+                                                                                                 key.p, N);
+  CKL();
+  k_dict_chunks<<<grid_for((int64_t)nc + 1, 256, 64), 256, 0, h->stream>>>(nc, CH, N, cstart.p, cq0.p, cnq.p);
+  CKL();
+  k_plan_hist<<<(nc + wpb - 1) / wpb, wpb * 32, sm, h->stream>>>(key.p, nullptr, cstart.p, cq0.p, cnq.p, nc, J, 1, H.p,
+                                                                  flag.p, N, 0);
+  CKL();
+  TRY(scan(H.p, (int64_t)J * nc));
+  k_plan_scatter<<<(nc + wpb - 1) / wpb, wpb * 32, sm, h->stream>>>(key.p, nullptr, cstart.p, cq0.p, cnq.p, nc, J, 1, H.p,
+                                                                     h->sort_perm.p, nullptr, nullptr, nullptr, N, 0, 0);
+  CKL();
+  k_dict_finish<<<grid_for(std::max<int64_t>(N, (int64_t)J + 1), 256, h->num_sms * 8), 256, 0, h->stream>>>(
+      h->sort_perm.p, h->inv_sort.p, N, H.p, nc, J, tst.p);
+  CKL();
+  std::vector<int> uniq_h(J), tst_h((size_t)J + 1);
+  CK(cudaMemcpyAsync(uniq_h.data(), uniq_d.p, sizeof(int) * (size_t)J, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(tst_h.data(), tst.p, sizeof(int) * ((size_t)J + 1), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  TRY(set_tuples(h, std::vector<uint64_t>(uniq_h.begin(), uniq_h.end()), radix));
+  tstart.assign(tst_h.begin(), tst_h.end());
+  // level counts: every level's tuples' cell counts, summed (integers, so the same numbers the host loop counts)
+  lvl_count.assign(B, 0);
+  for (int q = 0; q < J; ++q)
+    for (int c = 0; c < C; ++c) lvl_count[h->tuple_levels_h[(size_t)q * C + c]] += tstart[q + 1] - tstart[q];
+  if (h->world > 1) {
+    DevBuf<long long> dl;
+    CK(dl.alloc(B));
+    std::vector<long long> lc(lvl_count.begin(), lvl_count.end());
+    CK(cudaMemcpyAsync(dl.p, lc.data(), sizeof(long long) * B, cudaMemcpyHostToDevice, h->stream));
+    CKN(g_nccl.AllReduce(dl.p, dl.p, B, ncclInt64, ncclSum, h->comm, h->stream));
+    CK(cudaMemcpyAsync(lc.data(), dl.p, sizeof(long long) * B, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    lvl_count.assign(lc.begin(), lc.end());
+  }
+  return 0;
+}
+
+// (c) everything that follows from the tuple dictionary: tile and chunk tables, allocations, small uploads and the
+// CSR level -> tuple table
+int setup_tables(hb_handle* h, HostLap& lap, const std::vector<int64_t>& tstart, const std::vector<int64_t>& lvl_count,
+                 const double* sigma, const double* theta, const double* lambda) {
+  const int64_t N = h->n, NG = h->N_global;
+  const int J = h->J, B = h->B, C = h->C, K = h->K, d = h->d;
+  // static tiles (<= TM cells of one tuple) and plan chunks (<= CHUNK cells of one tuple)
+  int CHUNK = 1024;  // plan chunks: ~2000 per shard at most (the plan's scan is nb^2 x #chunks long)
+  while (CHUNK < 16384 && N / CHUNK > 2048) CHUNK <<= 1;
+  std::vector<int> t_cell0, t_len, t_tuple, c_start, t_chunk0(J, 0), c_q0, c_nq;
+  for (int q = 0; q < J; ++q) {
+    for (int64_t s = tstart[q]; s < tstart[q + 1]; s += TM) {
+      t_cell0.push_back((int)s);
+      t_len.push_back((int)std::min<int64_t>(TM, tstart[q + 1] - s));
+      t_tuple.push_back(q);
+    }
+    t_chunk0[q] = (int)c_start.size();
+    for (int64_t s = tstart[q]; s < tstart[q + 1]; s += CHUNK) c_start.push_back((int)s);
+    const int nq = (int)c_start.size() - t_chunk0[q];
+    for (int i = 0; i < nq; ++i) {
+      c_q0.push_back(t_chunk0[q]);
+      c_nq.push_back(nq);
+    }
+  }
+  std::vector<int> tc0, tcl, tct;  // 128-cell tiles for the tensor-core kernels
+  for (int q = 0; q < J; ++q)
+    for (int64_t s2 = tstart[q]; s2 < tstart[q + 1]; s2 += TC_TM) {
+      tc0.push_back((int)s2);
+      tcl.push_back((int)std::min<int64_t>(TC_TM, tstart[q + 1] - s2));
+      tct.push_back(q);
+    }
+  h->tc_ntiles = (int)tc0.size();
+  c_q0.push_back((int)c_start.size());  // the trailing empty chunk is a group of its own
+  c_nq.push_back(1);
+  c_start.push_back((int)N);  // start of the trailing empty chunk
+  c_start.push_back((int)N);  // and its end
+  h->ntiles = (int)t_cell0.size();
+  h->nchunks = (int)c_start.size() - 1;
+  // tuples without local cells point at the first later chunk (their segments are empty)
+  for (int q = J - 1; q >= 0; --q)
+    if (tstart[q + 1] == tstart[q]) t_chunk0[q] = (q + 1 < J) ? t_chunk0[q + 1] : h->nchunks - 1;
+
+  // ---- device allocations
+  const int KS = h->KS, DS = h->DS;
+  const size_t nK = (size_t)N * KS, nd = (size_t)N * DS, BK = (size_t)B * KS;
+  const int Tplan = std::max(1, (int)h->max_iter_kmeans);
+  // update_R kernels: the single-pass persistent kernel when every CTA's slice of a block can lie inside one
+  // covariate tuple (2 J <= #SMs) and its ring fits shared memory; else the first persistent generation (K <= 256,
+  // <= 8192 tuples, checked against the shared-memory limit); else one launch triple per block step.
+  const size_t smem_limit = (size_t)227 * 1024 - 256;
+  const bool force_v1 = (h->kernel_set & HB_KS_UPDATE_PER_STEP) != 0, force_v2 = (h->kernel_set & HB_KS_UPDATE_TWO_PASS) != 0;
+  h->coop_grid = h->num_sms;  // one persistent CTA per SM
+  h->aligned_ranges = (2 * J <= h->coop_grid);
+  h->u5_ring_rows = upd5_ring_rows(KS, smem_limit);
+  h->use_v4 = !force_v1 && !force_v2 && h->aligned_ranges && h->u5_ring_rows > 0 && (uint64_t)N * (uint64_t)KS < (1ull << 32);
+  h->use_v2 = h->use_v4 || (!force_v1 && (KS <= 256) && (J <= 8192) && upd_smem_bytes(h) <= smem_limit);
+  h->plan_nsub = (h->use_v4 && h->nb <= 64) ? h->nb : 1;
+  h->plan_rounds = Tplan;
+  CK(h->Zo.alloc(nd));
+  CK(h->Zc.alloc(nd));
+  CK(h->U.alloc(nK));
+  CK(h->R.alloc(nK));
+  CK(h->Y.alloc((size_t)K * d));
+  CK(h->sigma.alloc(K));
+  CK(h->theta.alloc(B));
+  CK(h->Pr_b.alloc(B));
+  CK(h->N_b.alloc(B));
+  CK(h->lambda.alloc(B + 1));
+  CK(h->O.alloc(BK));
+  CK(h->E.alloc(BK));
+  CK(h->P.alloc(BK));
+  CK(h->tmpT.alloc((size_t)B * K));
+  CK(h->Oacc.alloc(BK + KS));
+  CK(h->acc.alloc(4 * (BK + KS)));
+  CK(h->S.alloc((size_t)J * K * (d + 1)));
+  CK(h->V.alloc((size_t)J * K * d));
+  CK(h->Wfull.alloc((size_t)K * (B + 1) * d));
+  CK(h->scratch.alloc((size_t)K * (2 * (size_t)(B + 1) * (B + 1) + (size_t)(B + 1) * d)));
+  CK(h->iscratch.alloc((size_t)K * (2 * (size_t)B + J)));
+  CK(h->skipped.alloc(K));
+  CK(h->err_flag.alloc(1));
+  CK(h->obj_acc.alloc(2));
+  CK(h->stage.alloc((size_t)8 << 20));  // 64 MiB of doubles
+  CK(h->tuple_levels.alloc((size_t)J * C));
+  CK(h->cov_of_d.alloc(B));
+  CK(h->tile_cell0.alloc(h->ntiles));
+  CK(h->tile_len.alloc(h->ntiles));
+  CK(h->tile_tuple.alloc(h->ntiles));
+  CK(h->tc_cell0.alloc(h->tc_ntiles));
+  CK(h->tc_len.alloc(h->tc_ntiles));
+  CK(h->tc_tuple.alloc(h->tc_ntiles));
+  h->use_tc_apply = (d <= 128) && !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);   // cluster ranges of <= AP_MAXK per launch
+  h->use_tc_stats = !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);                  // 128 clusters x 64 columns per launch
+  h->assign_ns = assign3_smem_bytes(2, (d + 7) & ~7, (K + 15) & ~15, KS) <= smem_limit ? 2 : 1;
+  h->use_tc_assign = (d <= 64) && (K <= 128) && assign3_smem_bytes(h->assign_ns, (d + 7) & ~7, (K + 15) & ~15, KS) <= smem_limit &&
+                     !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);
+  h->use_tc_logits = !h->use_tc_assign && (d <= 128) && logits_smem_bytes((d + 7) & ~7) <= smem_limit &&
+                     !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);
+  h->pt_cap = (size_t)N / TC_TM + (size_t)h->nb * J + 2;
+  if (h->use_tc_assign && h->use_v4) {
+    CK(h->pt_p0.alloc(2 * h->pt_cap));
+    CK(h->pt_len.alloc(2 * h->pt_cap));
+    CK(h->pt_tuple.alloc(2 * h->pt_cap));
+    CK(h->pt_blk.alloc(2 * h->pt_cap));
+    CK(h->pt_count.alloc(2));
+    CK(h->pt_base.alloc((size_t)h->nb * J + 2));
+  }
+  CK(h->chunk_start.alloc(h->nchunks + 1));
+  CK(h->tuple_chunk0.alloc(J));
+  CK(h->blk_of.alloc(2 * (size_t)Tplan * N));
+  CK(h->order.alloc(2 * (size_t)Tplan * N));
+  if (h->use_v4)
+    CK(h->next_at.alloc(2 * (size_t)Tplan * N));
+  else
+    CK(h->prev_at.alloc(2 * (size_t)Tplan * N));
+  {  // histogram scratch of the plan's counting sort: as many rounds per launch as fit 64 MB (at most 8)
+    const size_t per_round = (size_t)h->nb * h->plan_nsub * h->nchunks;
+    h->plan_batch = (int)std::max<size_t>(1, std::min<size_t>({(size_t)8, (size_t)Tplan, ((size_t)16 << 20) / std::max<size_t>(1, per_round)}));
+    CK(h->H.alloc(per_round * h->plan_batch));
+    CK(h->scan_state.alloc((size_t)h->plan_batch * ((per_round + SCAN_TILE - 1) / SCAN_TILE + 1)));
+  }
+  CK(h->chunk_q0.alloc(h->nchunks));
+  CK(h->chunk_nq.alloc(h->nchunks));
+  CK(h->seg_start.alloc(2 * (size_t)Tplan * ((size_t)h->nb * J + 1)));
+  CK(h->tile_base.alloc(2 * (size_t)Tplan * ((size_t)h->nb * J + 1)));
+  if (h->use_v2) {
+    CK(h->ring.alloc(4 * BK));
+    CK(h->acc2.alloc(2 * (BK + KS) * ((size_t)Tplan * h->nb + 2)));
+    CK(h->Psave.alloc(h->use_v4 ? 1 : 2 * (size_t)h->nb * BK));
+    if (h->use_v4) CK(h->remT.alloc(2 * (size_t)h->nb * J * KS));
+    if (h->use_v4 && h->world > 1) CK(h->remS.alloc((size_t)h->nb * J * KS));
+    CK(h->OEend.alloc((size_t)Tplan * 2 * BK));
+    CK(h->obj2.alloc(2 * (size_t)Tplan));
+    CK(h->bar.alloc(2 * ((size_t)Tplan * h->nb + 2)));
+    if (h->aligned_ranges) CK(h->ranges.alloc(2 * (size_t)Tplan * h->nb * h->coop_grid));
+    release_peer_exchange(h);
+    if (h->use_v4 && h->world > 1 && h->world <= U4_MAXWORLD && !(h->kernel_set & HB_KS_NO_PEER_EXCHANGE))
+      TRY(setup_peer_exchange(h, Tplan));
+    if (const char* e = getenv("HB_TRACE_STEPS")) {
+      h->dbg_cta = atoi(e);
+      CK(h->dbg.alloc((size_t)(32 * h->nb + 2) * 16));
+      CK(cudaMemsetAsync(h->dbg.p, 0, sizeof(long long) * (size_t)(32 * h->nb + 2) * 16, h->stream));
+    }
+    CK(cudaMemsetAsync(h->Psave.p, 0, sizeof(float) * h->Psave.n, h->stream));
+    CK(cudaMemsetAsync(h->ring.p, 0, sizeof(float) * 4 * BK, h->stream));
+  }
+  lap.mark("device allocations");
+  CK(cudaMemsetAsync(h->err_flag.p, 0, sizeof(int), h->stream));
+  CK(cudaMemsetAsync(h->obj_acc.p, 0, 2 * sizeof(double), h->stream));
+  CK(cudaMemsetAsync(h->O.p, 0, sizeof(float) * BK, h->stream));
+  CK(cudaMemsetAsync(h->E.p, 0, sizeof(float) * BK, h->stream));
+  CK(cudaMemsetAsync(h->Wfull.p, 0, sizeof(float) * (size_t)K * (B + 1) * d, h->stream));
+  CK(cudaMemsetAsync(h->skipped.p, 0, sizeof(int) * K, h->stream));
+  CK(cudaMemsetAsync(h->R.p, 0, sizeof(float) * nK, h->stream));
+  CK(cudaMemsetAsync(h->Zo.p, 0, sizeof(float) * nd, h->stream));
+  CK(cudaMemsetAsync(h->Zc.p, 0, sizeof(float) * nd, h->stream));
+  k_fill_f<<<grid_for((int64_t)nK, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->U.p, (int64_t)nK, U_PAD);
+  CKL();
+  CK(cudaMemsetAsync(h->Y.p, 0, sizeof(float) * (size_t)K * d, h->stream));
+#define UP(buf, vec) CK(cudaMemcpyAsync(h->buf.p, (vec).data(), sizeof((vec)[0]) * (vec).size(), cudaMemcpyHostToDevice, h->stream))
+  UP(tuple_levels, h->tuple_levels_h);
+  // CSR level -> tuples containing it, ascending tuple order; trailing word: the number of levels of covariate 0
+  std::vector<int> lvl_ptr_h(B + 2, 0), lvl_tup_h((size_t)J * C);
+  {
+    for (size_t i = 0; i < h->tuple_levels_h.size(); ++i) lvl_ptr_h[h->tuple_levels_h[i] + 1]++;
+    for (int b = 0; b < B; ++b) lvl_ptr_h[b + 1] += lvl_ptr_h[b];
+    std::vector<int> fill(lvl_ptr_h.begin(), lvl_ptr_h.begin() + B);
+    for (int q = 0; q < J; ++q)
+      for (int c = 0; c < C; ++c) lvl_tup_h[fill[h->tuple_levels_h[(size_t)q * C + c]]++] = q;
+    lvl_ptr_h[B + 1] = h->B_vec[0];
+    CK(h->lvl_ptr.alloc(B + 2));
+    CK(h->lvl_tup.alloc(std::max<size_t>(1, lvl_tup_h.size())));
+    UP(lvl_ptr, lvl_ptr_h);
+    UP(lvl_tup, lvl_tup_h);
+  }
+  UP(cov_of_d, h->cov_of);
+  UP(tile_cell0, t_cell0);
+  UP(tile_len, t_len);
+  UP(tile_tuple, t_tuple);
+  UP(tc_cell0, tc0);
+  UP(tc_len, tcl);
+  UP(tc_tuple, tct);
+  UP(chunk_start, c_start);
+  UP(chunk_q0, c_q0);
+  UP(chunk_nq, c_nq);
+  UP(tuple_chunk0, t_chunk0);
+  {
+    std::vector<float> f(K);
+    for (int k = 0; k < K; ++k) f[k] = (float)sigma[k];
+    h->sigma0 = f[0];
+    h->sigma_uniform = true;
+    for (int k = 1; k < K; ++k) h->sigma_uniform = h->sigma_uniform && (f[k] == f[0]);
+    UP(sigma, f);
+    f.resize(B);
+    for (int b = 0; b < B; ++b) f[b] = (float)theta[b];
+    UP(theta, f);
+    std::vector<float> nbv(B), prb(B);
+    for (int b = 0; b < B; ++b) {
+      nbv[b] = (float)lvl_count[b];
+      prb[b] = (float)lvl_count[b] / (float)NG;  // harmony.cpp:67
+    }
+    UP(N_b, nbv);
+    UP(Pr_b, prb);
+    std::vector<float> lam(B + 1, 0.f);
+    if (!h->lambda_estimation)
+      for (int b = 0; b <= B; ++b) lam[b] = (float)lambda[b];
+    UP(lambda, lam);
+    CK(cudaStreamSynchronize(h->stream));
+  }
+#undef UP
+  lap.mark("memsets + small uploads");
+  return 0;
+}
+
+// The pointer is device (or managed) memory of the handle's device.
+int check_device_ptr(hb_handle* h, const void* p, const char* what) {
+  cudaPointerAttributes a;
+  if (!p) return fail(h, 2, "null argument");
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(h, 2, "%s is not CUDA device memory", what);
+  }
+  if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return fail(h, 2, "%s is not CUDA device memory", what);
+  if (a.device != h->device) return fail(h, 2, "%s is on CUDA device %d, the handle on device %d", what, a.device, h->device);
+  return 0;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1613,6 +2160,7 @@ int hb_create(hb_handle** out, int device) {
   cudaStreamCreateWithFlags(&h->plan_stream, cudaStreamNonBlocking);
   cudaEventCreateWithFlags(&h->plan_done, cudaEventDisableTiming);
   cudaEventCreateWithFlags(&h->ev0, cudaEventDisableTiming);
+  cudaEventCreateWithFlags(&h->io_ev, cudaEventDisableTiming);
   ensure_pinned_staging();  // process-wide; the first handle pays for it, not the first download
   keep_pool_memory(device);
   widen_pool();
@@ -1628,6 +2176,7 @@ void hb_destroy(hb_handle* h) {
   if (h->plan_done) cudaEventDestroy(h->plan_done);
   if (h->plan_stream) cudaStreamDestroy(h->plan_stream);
   if (h->ev0) cudaEventDestroy(h->ev0);
+  if (h->io_ev) cudaEventDestroy(h->io_ev);
   release_peer_exchange(h);
   cudaStream_t s = h->stream;
   delete h;  // frees device buffers
@@ -1710,388 +2259,55 @@ int hb_setup(hb_handle* h, const double* Z, int d, int64_t N, const int32_t* phi
              const double* sigma, const double* theta, const double* lambda, double alpha, int max_iter_kmeans,
              double epsilon_kmeans, double epsilon_harmony, int K, double block_size,
              double batch_proportion_cutoff, int verbose) {
-  if (!h) return 1;
-  if (h->ran_setup) return fail(h, 3, "setup was already run on this object");
-  if (!Z || !phi_i || !B_vec || !sigma || !theta) return fail(h, 2, "null argument");
-  if (d < 1 || N < 1 || C < 1 || K < 1) return fail(h, 2, "bad dimensions");
-  if (K > 1024) return fail(h, 2, "K = %d is not supported (K <= 1024)", K);
-  if (N > 2000000000LL) return fail(h, 2, "more than 2e9 cells per GPU are not supported");
-  CK(cudaSetDevice(h->device));
-  h->n = N;
-  if (!h->shard_set) {
-    if (h->world > 1) return fail(h, 3, "hb_set_shard is required when world_size > 1");
-    h->N_global = N;
-    h->cell_offset = 0;
-  }
-  const int64_t NG = h->N_global;
-  h->d = d;
-  h->C = C;
-  h->K = K;
-  h->KS = (K + 3) & ~3;
-  h->DS = (d + 3) & ~3;
-  h->B_vec.assign(B_vec, B_vec + C);
-  h->B = std::accumulate(h->B_vec.begin(), h->B_vec.end(), 0);
-  const int B = h->B;
-  h->cov_of.resize(B);
-  {
-    int b = 0;
-    for (int c = 0; c < C; ++c)
-      for (int l = 0; l < B_vec[c]; ++l) h->cov_of[b++] = c;
-  }
-  // harmony.cpp:83-91
-  if (NG < 6) return fail(h, 1, "Refusing to run with less than 6 cells");
-  if (NG < 40) {
-    h->warnings.push_back("Too few cells. Setting block_size to 0.2");
-    h->block_size = 0.2f;
-  } else {
-    h->block_size = (float)block_size;
-  }
-  h->epsilon_kmeans = (float)epsilon_kmeans;
-  h->epsilon_harmony = (float)epsilon_harmony;
-  h->alpha = (float)alpha;
-  h->cutoff = (float)batch_proportion_cutoff;
-  h->max_iter_kmeans = (unsigned)max_iter_kmeans;
-  h->verbose = verbose;
-  h->lambda_estimation = (lambda == nullptr) || (lambda[0] == -1);  // harmony.cpp:75
-  // update_R block geometry, harmony.cpp:280-281 (float arithmetic on the GLOBAL cell count)
-  h->nb = my_ceil(1.0f / h->block_size);
-  h->cpb = (uint32_t)((float)NG * h->block_size);
-  if (h->cpb == 0) return fail(h, 2, "block_size * N < 1");
-  {
-    int bits = 1;
-    while ((1ull << bits) < (uint64_t)NG) bits++;
-    h->half_bits = (bits + 1) / 2;
-  }
-
+  TRY(setup_scalars(h, Z, d, N, phi_i, B_vec, C, sigma, theta, lambda, alpha, max_iter_kmeans, epsilon_kmeans,
+                    epsilon_harmony, K, block_size, batch_proportion_cutoff, verbose));
   HostLap lap(h->stream, "hb_setup");
-  // ---- joint covariate tuples; cells get sorted by tuple (stable)
-  std::vector<int64_t> lvl_count(B, 0);
-  std::vector<uint64_t> key(N);
-  std::vector<uint64_t> radix(C);
-  {
-    long double prod = 1;
-    for (int c = 0; c < C; ++c) prod *= (long double)B_vec[c];
-    if (prod > 9e18L) return fail(h, 2, "covariate level product overflows 64 bits");
-    uint64_t r = 1;
-    for (int c = C - 1; c >= 0; --c) {
-      radix[c] = r;
-      r *= (uint64_t)B_vec[c];
-    }
-  }
-  {
-    std::vector<int> base(C, 0);
-    for (int c = 1; c < C; ++c) base[c] = base[c - 1] + B_vec[c - 1];
-    for (int64_t i = 0; i < N; ++i) {
-      uint64_t kk = 0;
-      for (int c = 0; c < C; ++c) {
-        int b = phi_i[i * C + c];
-        if (b < base[c] || b >= base[c] + B_vec[c]) return fail(h, 2, "phi row index %d of cell %lld is not a level of covariate %d", b, (long long)i, c);
-        lvl_count[b]++;
-        kk += (uint64_t)(b - base[c]) * radix[c];
-      }
-      key[i] = kk;
-    }
-  }
-  std::vector<uint64_t> uniq;
-  uint64_t key_space = 1;
-  for (int c = 0; c < C; ++c) key_space *= (uint64_t)B_vec[c];
-  const bool small_space = key_space <= (1ull << 22);  // the usual case: a direct table beats sorting N keys
-  if (small_space) {
-    std::vector<uint8_t> seen((size_t)key_space, 0);
-    for (int64_t i = 0; i < N; ++i) seen[key[i]] = 1;
-    for (uint64_t k2 = 0; k2 < key_space; ++k2)
-      if (seen[k2]) uniq.push_back(k2);
-  } else {
-    uniq = key;
-    std::sort(uniq.begin(), uniq.end());
-    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
-  }
-  if (h->world > 1) {
-    // global tuple dictionary = union over ranks; level counts summed over ranks
-    long long cnt = (long long)uniq.size(), maxcnt = 0;
-    DevBuf<long long> dcnt;
-    CK(dcnt.alloc(1));
-    CK(cudaMemcpyAsync(dcnt.p, &cnt, sizeof(cnt), cudaMemcpyHostToDevice, h->stream));
-    CKN(g_nccl.AllReduce(dcnt.p, dcnt.p, 1, ncclInt64, ncclMax, h->comm, h->stream));
-    CK(cudaMemcpyAsync(&maxcnt, dcnt.p, sizeof(cnt), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    std::vector<uint64_t> sendbuf((size_t)maxcnt, ~0ull), recvbuf((size_t)maxcnt * h->world);
-    std::copy(uniq.begin(), uniq.end(), sendbuf.begin());
-    DevBuf<uint64_t> ds, dr;
-    CK(ds.alloc((size_t)maxcnt));
-    CK(dr.alloc((size_t)maxcnt * h->world));
-    CK(cudaMemcpyAsync(ds.p, sendbuf.data(), sizeof(uint64_t) * (size_t)maxcnt, cudaMemcpyHostToDevice, h->stream));
-    CKN(g_nccl.AllGather(ds.p, dr.p, (size_t)maxcnt, ncclUint64, h->comm, h->stream));
-    CK(cudaMemcpyAsync(recvbuf.data(), dr.p, sizeof(uint64_t) * recvbuf.size(), cudaMemcpyDeviceToHost, h->stream));
-    DevBuf<long long> dl;
-    CK(dl.alloc(B));
-    std::vector<long long> lc(lvl_count.begin(), lvl_count.end());
-    CK(cudaMemcpyAsync(dl.p, lc.data(), sizeof(long long) * B, cudaMemcpyHostToDevice, h->stream));
-    CKN(g_nccl.AllReduce(dl.p, dl.p, B, ncclInt64, ncclSum, h->comm, h->stream));
-    CK(cudaMemcpyAsync(lc.data(), dl.p, sizeof(long long) * B, cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    for (int b = 0; b < B; ++b) lvl_count[b] = lc[b];
-    uniq.assign(recvbuf.begin(), recvbuf.end());
-    std::sort(uniq.begin(), uniq.end());
-    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
-    if (!uniq.empty() && uniq.back() == ~0ull) uniq.pop_back();
-  }
-  if (uniq.size() > 1000000) return fail(h, 2, "more than 1e6 distinct covariate tuples are not supported");
-  const int J = (int)uniq.size();
-  h->J = J;
-  h->tuple_levels_h.resize((size_t)J * C);
-  {
-    std::vector<int> base(C, 0);
-    for (int c = 1; c < C; ++c) base[c] = base[c - 1] + B_vec[c - 1];
-    for (int q = 0; q < J; ++q) {
-      uint64_t kk = uniq[q];
-      for (int c = 0; c < C; ++c) {
-        h->tuple_levels_h[(size_t)q * C + c] = base[c] + (int)(kk / radix[c]);
-        kk %= radix[c];
-      }
-    }
-  }
-  std::vector<int> tuple_of(N);
-  std::vector<int64_t> tstart(J + 1, 0);
-  {
-    std::vector<int> lut;
-    if (small_space) {
-      lut.assign((size_t)key_space, -1);
-      for (int q = 0; q < J; ++q) lut[uniq[q]] = q;
-    }
-    for (int64_t i = 0; i < N; ++i) {
-      int q = small_space ? lut[key[i]] : (int)(std::lower_bound(uniq.begin(), uniq.end(), key[i]) - uniq.begin());
-      tuple_of[i] = q;
-      tstart[q + 1]++;
-    }
-  }
-  for (int q = 0; q < J; ++q) tstart[q + 1] += tstart[q];
-  h->sort_perm_h.resize(N);
-  std::vector<int> inv_sort(N);
-  {
-    std::vector<int64_t> cur(tstart.begin(), tstart.end() - 1);
-    for (int64_t i = 0; i < N; ++i) {
-      int64_t s = cur[tuple_of[i]]++;
-      h->sort_perm_h[s] = (int)i;
-      inv_sort[i] = (int)s;
-    }
-  }
-  // static tiles (<= TM cells of one tuple) and plan chunks (<= CHUNK cells of one tuple)
-  int CHUNK = 1024;  // plan chunks: ~2000 per shard at most (the plan's scan is nb^2 x #chunks long)
-  while (CHUNK < 16384 && N / CHUNK > 2048) CHUNK <<= 1;
-  std::vector<int> t_cell0, t_len, t_tuple, c_start, t_chunk0(J, 0), c_q0, c_nq;
-  for (int q = 0; q < J; ++q) {
-    for (int64_t s = tstart[q]; s < tstart[q + 1]; s += TM) {
-      t_cell0.push_back((int)s);
-      t_len.push_back((int)std::min<int64_t>(TM, tstart[q + 1] - s));
-      t_tuple.push_back(q);
-    }
-    t_chunk0[q] = (int)c_start.size();
-    for (int64_t s = tstart[q]; s < tstart[q + 1]; s += CHUNK) c_start.push_back((int)s);
-    const int nq = (int)c_start.size() - t_chunk0[q];
-    for (int i = 0; i < nq; ++i) {
-      c_q0.push_back(t_chunk0[q]);
-      c_nq.push_back(nq);
-    }
-  }
-  std::vector<int> tc0, tcl, tct;  // 128-cell tiles for the tensor-core kernels
-  for (int q = 0; q < J; ++q)
-    for (int64_t s2 = tstart[q]; s2 < tstart[q + 1]; s2 += TC_TM) {
-      tc0.push_back((int)s2);
-      tcl.push_back((int)std::min<int64_t>(TC_TM, tstart[q + 1] - s2));
-      tct.push_back(q);
-    }
-  h->tc_ntiles = (int)tc0.size();
-  c_q0.push_back((int)c_start.size());  // the trailing empty chunk is a group of its own
-  c_nq.push_back(1);
-  c_start.push_back((int)N);  // start of the trailing empty chunk
-  c_start.push_back((int)N);  // and its end
-  h->ntiles = (int)t_cell0.size();
-  h->nchunks = (int)c_start.size() - 1;
-  // tuples without local cells point at the first later chunk (their segments are empty)
-  for (int q = J - 1; q >= 0; --q)
-    if (tstart[q + 1] == tstart[q]) t_chunk0[q] = (q + 1 < J) ? t_chunk0[q + 1] : h->nchunks - 1;
-
+  std::vector<int64_t> lvl_count, tstart;
+  TRY(tuple_dict_host(h, phi_i, lvl_count, tstart));
   lap.mark("tuple dictionary / sort (host)");
-  // ---- device allocations
-  const int KS = h->KS, DS = h->DS;
-  const size_t nK = (size_t)N * KS, nd = (size_t)N * DS, BK = (size_t)B * KS;
-  const int Tplan = std::max(1, (int)h->max_iter_kmeans);
-  // update_R kernels: the single-pass persistent kernel when every CTA's slice of a block can lie inside one
-  // covariate tuple (2 J <= #SMs) and its ring fits shared memory; else the first persistent generation (K <= 256,
-  // <= 8192 tuples, checked against the shared-memory limit); else one launch triple per block step.
-  const size_t smem_limit = (size_t)227 * 1024 - 256;
-  const bool force_v1 = (h->kernel_set & HB_KS_UPDATE_PER_STEP) != 0, force_v2 = (h->kernel_set & HB_KS_UPDATE_TWO_PASS) != 0;
-  h->coop_grid = h->num_sms;  // one persistent CTA per SM
-  h->aligned_ranges = (2 * J <= h->coop_grid);
-  h->u5_ring_rows = upd5_ring_rows(KS, smem_limit);
-  h->use_v4 = !force_v1 && !force_v2 && h->aligned_ranges && h->u5_ring_rows > 0 && (uint64_t)N * (uint64_t)KS < (1ull << 32);
-  h->use_v2 = h->use_v4 || (!force_v1 && (KS <= 256) && (J <= 8192) && upd_smem_bytes(h) <= smem_limit);
-  h->plan_nsub = (h->use_v4 && h->nb <= 64) ? h->nb : 1;
-  h->plan_rounds = Tplan;
-  CK(h->Zo.alloc(nd));
-  CK(h->Zc.alloc(nd));
-  CK(h->U.alloc(nK));
-  CK(h->R.alloc(nK));
-  CK(h->Y.alloc((size_t)K * d));
-  CK(h->sigma.alloc(K));
-  CK(h->theta.alloc(B));
-  CK(h->Pr_b.alloc(B));
-  CK(h->N_b.alloc(B));
-  CK(h->lambda.alloc(B + 1));
-  CK(h->O.alloc(BK));
-  CK(h->E.alloc(BK));
-  CK(h->P.alloc(BK));
-  CK(h->tmpT.alloc((size_t)B * K));
-  CK(h->Oacc.alloc(BK + KS));
-  CK(h->acc.alloc(4 * (BK + KS)));
-  CK(h->S.alloc((size_t)J * K * (d + 1)));
-  CK(h->V.alloc((size_t)J * K * d));
-  CK(h->Wfull.alloc((size_t)K * (B + 1) * d));
-  CK(h->scratch.alloc((size_t)K * (2 * (size_t)(B + 1) * (B + 1) + (size_t)(B + 1) * d)));
-  CK(h->iscratch.alloc((size_t)K * (2 * (size_t)B + J)));
-  CK(h->skipped.alloc(K));
-  CK(h->err_flag.alloc(1));
-  CK(h->obj_acc.alloc(2));
-  CK(h->stage.alloc((size_t)8 << 20));  // 64 MiB of doubles
-  CK(h->sort_perm.alloc(N));
-  CK(h->inv_sort.alloc(N));
-  CK(h->tuple_levels.alloc((size_t)J * C));
-  CK(h->cov_of_d.alloc(B));
-  CK(h->tile_cell0.alloc(h->ntiles));
-  CK(h->tile_len.alloc(h->ntiles));
-  CK(h->tile_tuple.alloc(h->ntiles));
-  CK(h->tc_cell0.alloc(h->tc_ntiles));
-  CK(h->tc_len.alloc(h->tc_ntiles));
-  CK(h->tc_tuple.alloc(h->tc_ntiles));
-  h->use_tc_apply = (d <= 128) && !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);   // cluster ranges of <= AP_MAXK per launch
-  h->use_tc_stats = !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);                  // 128 clusters x 64 columns per launch
-  h->assign_ns = assign3_smem_bytes(2, (d + 7) & ~7, (K + 15) & ~15, KS) <= smem_limit ? 2 : 1;
-  h->use_tc_assign = (d <= 64) && (K <= 128) && assign3_smem_bytes(h->assign_ns, (d + 7) & ~7, (K + 15) & ~15, KS) <= smem_limit &&
-                     !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);
-  h->use_tc_logits = !h->use_tc_assign && (d <= 128) && logits_smem_bytes((d + 7) & ~7) <= smem_limit &&
-                     !(h->kernel_set & HB_KS_FFMA_CONTRACTIONS);
-  h->pt_cap = (size_t)N / TC_TM + (size_t)h->nb * J + 2;
-  if (h->use_tc_assign && h->use_v4) {
-    CK(h->pt_p0.alloc(2 * h->pt_cap));
-    CK(h->pt_len.alloc(2 * h->pt_cap));
-    CK(h->pt_tuple.alloc(2 * h->pt_cap));
-    CK(h->pt_blk.alloc(2 * h->pt_cap));
-    CK(h->pt_count.alloc(2));
-    CK(h->pt_base.alloc((size_t)h->nb * J + 2));
-  }
-  CK(h->chunk_start.alloc(h->nchunks + 1));
-  CK(h->tuple_chunk0.alloc(J));
-  CK(h->blk_of.alloc(2 * (size_t)Tplan * N));
-  CK(h->order.alloc(2 * (size_t)Tplan * N));
-  if (h->use_v4)
-    CK(h->next_at.alloc(2 * (size_t)Tplan * N));
-  else
-    CK(h->prev_at.alloc(2 * (size_t)Tplan * N));
-  {  // histogram scratch of the plan's counting sort: as many rounds per launch as fit 64 MB (at most 8)
-    const size_t per_round = (size_t)h->nb * h->plan_nsub * h->nchunks;
-    h->plan_batch = (int)std::max<size_t>(1, std::min<size_t>({(size_t)8, (size_t)Tplan, ((size_t)16 << 20) / std::max<size_t>(1, per_round)}));
-    CK(h->H.alloc(per_round * h->plan_batch));
-    CK(h->scan_state.alloc((size_t)h->plan_batch * ((per_round + SCAN_TILE - 1) / SCAN_TILE + 1)));
-  }
-  CK(h->chunk_q0.alloc(h->nchunks));
-  CK(h->chunk_nq.alloc(h->nchunks));
-  CK(h->seg_start.alloc(2 * (size_t)Tplan * ((size_t)h->nb * J + 1)));
-  CK(h->tile_base.alloc(2 * (size_t)Tplan * ((size_t)h->nb * J + 1)));
-  if (h->use_v2) {
-    CK(h->ring.alloc(4 * BK));
-    CK(h->acc2.alloc(2 * (BK + KS) * ((size_t)Tplan * h->nb + 2)));
-    CK(h->Psave.alloc(h->use_v4 ? 1 : 2 * (size_t)h->nb * BK));
-    if (h->use_v4) CK(h->remT.alloc(2 * (size_t)h->nb * J * KS));
-    if (h->use_v4 && h->world > 1) CK(h->remS.alloc((size_t)h->nb * J * KS));
-    CK(h->OEend.alloc((size_t)Tplan * 2 * BK));
-    CK(h->obj2.alloc(2 * (size_t)Tplan));
-    CK(h->bar.alloc(2 * ((size_t)Tplan * h->nb + 2)));
-    if (h->aligned_ranges) CK(h->ranges.alloc(2 * (size_t)Tplan * h->nb * h->coop_grid));
-    release_peer_exchange(h);
-    if (h->use_v4 && h->world > 1 && h->world <= U4_MAXWORLD && !(h->kernel_set & HB_KS_NO_PEER_EXCHANGE))
-      TRY(setup_peer_exchange(h, Tplan));
-    if (const char* e = getenv("HB_TRACE_STEPS")) {
-      h->dbg_cta = atoi(e);
-      CK(h->dbg.alloc((size_t)(32 * h->nb + 2) * 16));
-      CK(cudaMemsetAsync(h->dbg.p, 0, sizeof(long long) * (size_t)(32 * h->nb + 2) * 16, h->stream));
-    }
-    CK(cudaMemsetAsync(h->Psave.p, 0, sizeof(float) * h->Psave.n, h->stream));
-    CK(cudaMemsetAsync(h->ring.p, 0, sizeof(float) * 4 * BK, h->stream));
-  }
-  lap.mark("device allocations");
-  CK(cudaMemsetAsync(h->err_flag.p, 0, sizeof(int), h->stream));
-  CK(cudaMemsetAsync(h->obj_acc.p, 0, 2 * sizeof(double), h->stream));
-  CK(cudaMemsetAsync(h->O.p, 0, sizeof(float) * BK, h->stream));
-  CK(cudaMemsetAsync(h->E.p, 0, sizeof(float) * BK, h->stream));
-  CK(cudaMemsetAsync(h->Wfull.p, 0, sizeof(float) * (size_t)K * (B + 1) * d, h->stream));
-  CK(cudaMemsetAsync(h->skipped.p, 0, sizeof(int) * K, h->stream));
-  CK(cudaMemsetAsync(h->R.p, 0, sizeof(float) * nK, h->stream));
-  CK(cudaMemsetAsync(h->Zo.p, 0, sizeof(float) * nd, h->stream));
-  CK(cudaMemsetAsync(h->Zc.p, 0, sizeof(float) * nd, h->stream));
-  k_fill_f<<<grid_for((int64_t)nK, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->U.p, (int64_t)nK, U_PAD);
-  CKL();
-  CK(cudaMemsetAsync(h->Y.p, 0, sizeof(float) * (size_t)K * d, h->stream));
-#define UP(buf, vec) CK(cudaMemcpyAsync(h->buf.p, (vec).data(), sizeof((vec)[0]) * (vec).size(), cudaMemcpyHostToDevice, h->stream))
-  UP(sort_perm, h->sort_perm_h);
-  UP(inv_sort, inv_sort);
-  UP(tuple_levels, h->tuple_levels_h);
-  // CSR level -> tuples containing it, ascending tuple order; trailing word: the number of levels of covariate 0
-  std::vector<int> lvl_ptr_h(B + 2, 0), lvl_tup_h((size_t)J * C);
-  {
-    for (size_t i = 0; i < h->tuple_levels_h.size(); ++i) lvl_ptr_h[h->tuple_levels_h[i] + 1]++;
-    for (int b = 0; b < B; ++b) lvl_ptr_h[b + 1] += lvl_ptr_h[b];
-    std::vector<int> fill(lvl_ptr_h.begin(), lvl_ptr_h.begin() + B);
-    for (int q = 0; q < J; ++q)
-      for (int c = 0; c < C; ++c) lvl_tup_h[fill[h->tuple_levels_h[(size_t)q * C + c]]++] = q;
-    lvl_ptr_h[B + 1] = h->B_vec[0];
-    CK(h->lvl_ptr.alloc(B + 2));
-    CK(h->lvl_tup.alloc(std::max<size_t>(1, lvl_tup_h.size())));
-    UP(lvl_ptr, lvl_ptr_h);
-    UP(lvl_tup, lvl_tup_h);
-  }
-  UP(cov_of_d, h->cov_of);
-  UP(tile_cell0, t_cell0);
-  UP(tile_len, t_len);
-  UP(tile_tuple, t_tuple);
-  UP(tc_cell0, tc0);
-  UP(tc_len, tcl);
-  UP(tc_tuple, tct);
-  UP(chunk_start, c_start);
-  UP(chunk_q0, c_q0);
-  UP(chunk_nq, c_nq);
-  UP(tuple_chunk0, t_chunk0);
-  {
-    std::vector<float> f(K);
-    for (int k = 0; k < K; ++k) f[k] = (float)sigma[k];
-    h->sigma0 = f[0];
-    h->sigma_uniform = true;
-    for (int k = 1; k < K; ++k) h->sigma_uniform = h->sigma_uniform && (f[k] == f[0]);
-    UP(sigma, f);
-    f.resize(B);
-    for (int b = 0; b < B; ++b) f[b] = (float)theta[b];
-    UP(theta, f);
-    std::vector<float> nbv(B), prb(B);
-    for (int b = 0; b < B; ++b) {
-      nbv[b] = (float)lvl_count[b];
-      prb[b] = (float)lvl_count[b] / (float)NG;  // harmony.cpp:67
-    }
-    UP(N_b, nbv);
-    UP(Pr_b, prb);
-    std::vector<float> lam(B + 1, 0.f);
-    if (!h->lambda_estimation)
-      for (int b = 0; b <= B; ++b) lam[b] = (float)lambda[b];
-    UP(lambda, lam);
-    CK(cudaStreamSynchronize(h->stream));
-  }
-#undef UP
-  lap.mark("memsets + small uploads");
+  TRY(setup_tables(h, lap, tstart, lvl_count, sigma, theta, lambda));
   // Z: double -> float, into tuple-sorted order (harmony.cpp:41); Z_corr = normalise(Z_orig) (:42)
   TRY(upload_rows(h, Z, d, h->DS, h->Zo.p));
   k_normalise_rows<<<grid_for(N * 32, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->Zo.p, h->Zc.p, N, d, h->DS);
   CKL();
   CK(cudaStreamSynchronize(h->stream));
   lap.mark("Z upload + normalise");
+  h->ran_setup = true;
+  return 0;
+}
+
+int hb_setup_device(hb_handle* h, const void* Z, int z_dtype, int64_t z_cell_stride, int64_t z_pc_stride, int d,
+                    int64_t N, const int32_t* phi_i, const int32_t* B_vec, int C, const double* sigma,
+                    const double* theta, const double* lambda, double alpha, int max_iter_kmeans,
+                    double epsilon_kmeans, double epsilon_harmony, int K, double block_size,
+                    double batch_proportion_cutoff, int verbose, void* stream) {
+  TRY(setup_scalars(h, Z, d, N, phi_i, B_vec, C, sigma, theta, lambda, alpha, max_iter_kmeans, epsilon_kmeans,
+                    epsilon_harmony, K, block_size, batch_proportion_cutoff, verbose));
+  if (z_dtype != HB_F32 && z_dtype != HB_F64) return fail(h, 2, "Z dtype %d is not supported (HB_F32 or HB_F64)", z_dtype);
+  if (z_cell_stride < 0 || z_pc_stride < 0) return fail(h, 2, "negative Z strides are not supported");
+  TRY(check_device_ptr(h, Z, "Z"));
+  TRY(check_device_ptr(h, phi_i, "phi_i"));
+  HostLap lap(h->stream, "hb_setup_device");
+  // Z and phi_i are ready on the caller's stream: this handle's stream waits for it
+  CK(cudaEventRecord(h->io_ev, (cudaStream_t)stream));
+  CK(cudaStreamWaitEvent(h->stream, h->io_ev, 0));
+  std::vector<int64_t> lvl_count, tstart;
+  TRY(tuple_dict_device(h, phi_i, lvl_count, tstart));
+  lap.mark("tuple dictionary / sort (device)");
+  TRY(setup_tables(h, lap, tstart, lvl_count, sigma, theta, lambda));
+  // the host path's conversion and scatter, read straight from the caller's layout
+  const int grid = grid_for(N * d, 256, h->num_sms * 8);
+  if (z_dtype == HB_F32)
+    k_upload_rows<<<grid, 256, 0, h->stream>>>(static_cast<const float*>(Z), z_cell_stride, z_pc_stride, h->Zo.p,
+                                               h->inv_sort.p, 0, N, d, h->DS);
+  else
+    k_upload_rows<<<grid, 256, 0, h->stream>>>(static_cast<const double*>(Z), z_cell_stride, z_pc_stride, h->Zo.p,
+                                               h->inv_sort.p, 0, N, d, h->DS);
+  CKL();
+  k_normalise_rows<<<grid_for(N * 32, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->Zo.p, h->Zc.p, N, d, h->DS);
+  CKL();
+  CK(cudaStreamSynchronize(h->stream));  // the inputs are consumed: the caller may free them
+  lap.mark("Z ingest + normalise");
   h->ran_setup = true;
   return 0;
 }
@@ -2556,6 +2772,47 @@ int hb_get_field(hb_handle* h, int field, double* out) {
   return fail(h, 2, "unknown field %d", field);
 }
 
+int hb_get_field_device(hb_handle* h, int field, void* out, int dtype, int64_t ld, void* stream) {
+  if (!h) return 1;
+  if (!h->ran_setup) return fail(h, 3, "setup has not been run");
+  if (dtype != HB_F32 && dtype != HB_F64) return fail(h, 2, "output dtype %d is not supported (HB_F32 or HB_F64)", dtype);
+  const float* src = nullptr;
+  int cols = 0, sld = 0;
+  switch (field) {
+    case HB_Z_CORR: src = h->Zc.p, cols = h->d, sld = h->DS; break;
+    case HB_Z_ORIG: src = h->Zo.p, cols = h->d, sld = h->DS; break;
+    case HB_R: src = h->R.p, cols = h->K, sld = h->KS; break;
+    default: return fail(h, 2, "field %d is not a per-cell field", field);
+  }
+  if (ld < cols) return fail(h, 2, "row stride %lld is shorter than a row (%d values)", (long long)ld, cols);
+  TRY(check_device_ptr(h, out, "out"));
+  CK(cudaSetDevice(h->device));
+  CK(cudaEventRecord(h->io_ev, (cudaStream_t)stream));  // the caller's earlier use of `out` ...
+  CK(cudaStreamWaitEvent(h->stream, h->io_ev, 0));      // ... precedes the write
+  if (field == HB_Z_CORR && h->zc_pending_norm) {  // as hb_get_field
+    k_normalise_rows<<<grid_for((int64_t)h->n * 32, 256, h->num_sms * 8), 256, 0, h->stream>>>(h->Zc.p, h->Zc.p, h->n, h->d, h->DS);
+    CKL();
+    h->zc_pending_norm = false;
+  }
+  const int grid = grid_for(h->n * cols, 256, h->num_sms * 8);
+  if (dtype == HB_F32)
+    k_download_rows<<<grid, 256, 0, h->stream>>>(src, static_cast<float*>(out), ld, h->inv_sort.p, 0, h->n, cols, sld);
+  else
+    k_download_rows<<<grid, 256, 0, h->stream>>>(src, static_cast<double*>(out), ld, h->inv_sort.p, 0, h->n, cols, sld);
+  CKL();
+  CK(cudaEventRecord(h->io_ev, h->stream));  // the caller's stream reads `out` after the write
+  CK(cudaStreamWaitEvent((cudaStream_t)stream, h->io_ev, 0));
+  return 0;
+}
+
+int hb_debug_sort_perm(const hb_handle* h, int32_t* out) {
+  if (!h || !out || !h->ran_setup) return 1;
+  if (cudaSetDevice(h->device) != cudaSuccess || cudaStreamSynchronize(h->stream) != cudaSuccess ||
+      cudaMemcpy(out, h->sort_perm.p, sizeof(int32_t) * (size_t)h->n, cudaMemcpyDeviceToHost) != cudaSuccess)
+    return 10;
+  return 0;
+}
+
 int hb_set_field(hb_handle* h, int field, const double* in) {
   if (!h) return 1;
   if (!h->ran_setup) return fail(h, 3, "setup has not been run");
@@ -2603,6 +2860,7 @@ int hb_get_scalar(const hb_handle* h, int which, double* out) {
     case HB_WINDOW_SIZE: *out = h->window_size; return 0;
     case HB_LEGACY_CENTROID_STEP: *out = h->legacy_centroid ? 1 : 0; return 0;
     case HB_KERNEL_SET: *out = h->kernel_set; return 0;
+    case HB_DEVICE: *out = h->device; return 0;
   }
   return 2;
 }

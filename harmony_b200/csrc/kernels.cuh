@@ -21,27 +21,40 @@ constexpr int NWARP = ROW_THREADS / 32;
 // ------------------------------------------------------------------------------------------------
 // setup helpers
 // ------------------------------------------------------------------------------------------------
-// dst[dst_row[r0 + r]][c] = (float)src[r][c]   (double -> float conversion of harmony.cpp:41 fused
-// with the scatter into tuple-sorted order)
-__global__ void k_upload_rows(const double* __restrict__ src, float* __restrict__ dst,
+// dst[dst_row[r0 + r]][c] = (float)src[r * src_rs + c * src_cs]   (double / float -> float conversion of
+// harmony.cpp:41 fused with the scatter into tuple-sorted order).  Strides in elements: (cols, 1) for the host path's
+// staging rows, any pair for a caller's device tensor; consecutive threads walk the source's smaller stride.
+template <typename T>
+__global__ void k_upload_rows(const T* __restrict__ src, int64_t src_rs, int64_t src_cs, float* __restrict__ dst,
                               const int* __restrict__ dst_row, int64_t r0, int64_t rows, int cols, int ld) {
+  const bool along_row = src_cs <= src_rs;
   int64_t total = rows * cols;
   for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total;
        idx += (int64_t)gridDim.x * blockDim.x) {
-    int64_t r = idx / cols;
-    int c = (int)(idx - r * cols);
-    dst[(int64_t)dst_row[r0 + r] * ld + c] = (float)src[idx];
+    int64_t r;
+    int c;
+    if (along_row) {
+      r = idx / cols;
+      c = (int)(idx - r * cols);
+    } else {
+      c = (int)(idx / rows);
+      r = idx - (int64_t)c * rows;
+    }
+    dst[(int64_t)dst_row[r0 + r] * ld + c] = (float)src[r * src_rs + (int64_t)c * src_cs];
   }
 }
-// out[r][c] = (double) src[src_row[r0 + r]][c]   (conv_to<RMAT>::from of harmony.cpp:640-650 + un-sort)
-__global__ void k_download_rows(const float* __restrict__ src, double* __restrict__ out,
+// out[r * out_ld + c] = (T) src[src_row[r0 + r]][c]   (conv_to<RMAT>::from of harmony.cpp:640-650 + un-sort).  T = double:
+// the host path's staging rows; T = float: its threaded variant (the host workers widen while they scatter) and
+// device outputs of either type.
+template <typename T>
+__global__ void k_download_rows(const float* __restrict__ src, T* __restrict__ out, int64_t out_ld,
                                 const int* __restrict__ src_row, int64_t r0, int64_t rows, int cols, int ld) {
   int64_t total = rows * cols;
   for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total;
        idx += (int64_t)gridDim.x * blockDim.x) {
     int64_t r = idx / cols;
     int c = (int)(idx - r * cols);
-    out[idx] = (double)src[(int64_t)src_row[r0 + r] * ld + c];
+    out[r * out_ld + c] = (T)src[(int64_t)src_row[r0 + r] * ld + c];
   }
 }
 // Legacy centroid step (harmony.cpp:235-238, commented out in 2.0.4): Y_k = normalise(sum_i R_ik z_i) from the
@@ -60,17 +73,6 @@ __global__ void k_centroids_from_stats(const float* __restrict__ S, float* __res
   float nrm = sqrtf(ss);
   if (nrm == 0.f) nrm = 1.f;
   for (int c = threadIdx.x; c < d; c += blockDim.x) Y[(size_t)k * d + c] = ysum[c] / nrm;
-}
-// float variant for the threaded download path (the host workers widen to double while they scatter)
-__global__ void k_download_rows_f(const float* __restrict__ src, float* __restrict__ out, const int* __restrict__ src_row,
-                                  int64_t r0, int64_t rows, int cols, int ld) {
-  int64_t total = rows * cols;
-  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total;
-       idx += (int64_t)gridDim.x * blockDim.x) {
-    int64_t r = idx / cols;
-    int c = (int)(idx - r * cols);
-    out[idx] = src[(int64_t)src_row[r0 + r] * ld + c];
-  }
 }
 __global__ void k_fill_f(float* __restrict__ out, int64_t n, float v) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = v;

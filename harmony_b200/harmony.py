@@ -8,6 +8,7 @@ Shapes follow R (column-major, cells are columns): ``obj.R`` is [K, N], ``obj.ge
 C ABI fills, i.e. the bytes an R numeric matrix would hold.
 """
 import ctypes
+import sys
 import warnings
 
 import numpy as np
@@ -18,10 +19,12 @@ FIELD = {"Z_corr": 0, "Z_orig": 1, "R": 2, "Y": 3, "O": 4, "E": 5, "W": 6, "Pr_b
          "lambda_mat": 10, "lambda": 11}
 SCALAR = {"N": 0, "B": 1, "K": 2, "d": 3, "C": 4, "alpha": 5, "max_iter_kmeans": 6, "block_size": 7,
           "epsilon_kmeans": 8, "epsilon_harmony": 9, "N_local": 10, "lambda_estimation": 11, "window_size": 12,
-          "legacy_centroid_step": 13, "kernel_set": 14}
+          "legacy_centroid_step": 13, "kernel_set": 14, "device": 15}
 TRACE = {"objective_kmeans": 0, "objective_kmeans_dist": 1, "objective_kmeans_entropy": 2,
          "objective_kmeans_cross": 3, "objective_harmony": 4, "kmeans_rounds": 5}
-_INT_SCALARS = ("N", "B", "K", "d", "C", "max_iter_kmeans", "N_local", "window_size", "legacy_centroid_step", "kernel_set")
+_INT_SCALARS = ("N", "B", "K", "d", "C", "max_iter_kmeans", "N_local", "window_size", "legacy_centroid_step", "kernel_set",
+                "device")
+HB_F32, HB_F64 = 0, 1   # enum hb_dtype
 
 
 def _ptr(a):
@@ -30,6 +33,47 @@ def _ptr(a):
 
 class HarmonyError(RuntimeError):
     pass
+
+
+def torch_of(x):
+    """The torch module if ``x`` is a ``torch.Tensor``, else None.  Never imports torch: a caller that passes numpy
+    arrays does not pay for it, and a tensor cannot exist unless torch was imported already."""
+    torch = sys.modules.get("torch")
+    return torch if torch is not None and isinstance(x, torch.Tensor) else None
+
+
+def tensor_abi_args(Z, n):
+    """(dtype code, cell stride, PC stride, d) of hb_setup_device for a 2-D float tensor ``Z`` of ``n`` cells, given as
+    [n, d] or [d, n] (the same orientation rule as numpy input), any strides; strides are in elements."""
+    torch = torch_of(Z)
+    if Z.dim() != 2:
+        raise ValueError(f"Z must be a 2-D tensor (cells x PCs or PCs x cells), not {Z.dim()}-D")
+    codes = {torch.float32: HB_F32, torch.float64: HB_F64}
+    if Z.dtype not in codes:
+        raise TypeError(f"Z must be float32 or float64, not {Z.dtype}")
+    if Z.shape[0] != n and Z.shape[1] == n:
+        Z = Z.T
+    if Z.shape[0] != n:
+        raise ValueError("number of cells in Z and Phi differ")
+    return codes[Z.dtype], int(Z.stride(0)), int(Z.stride(1)), int(Z.shape[1])
+
+
+def _setup_params(sigma, theta, lambda_, K, B_vec):
+    """Host-side scalars of harmony::setup as the C ABI takes them: (B_vec, K, sigma, theta, lambda or None)."""
+    B_vec = np.ascontiguousarray(np.atleast_1d(B_vec), dtype=np.int32)
+    K = int(K)
+    sigma = np.ascontiguousarray(np.broadcast_to(np.asarray(sigma, dtype=np.float64), (K,)))
+    theta = np.ascontiguousarray(theta, dtype=np.float64)
+    if len(theta) != int(B_vec.sum()):
+        raise ValueError("theta must hold one value per covariate level")
+    lam = None
+    if lambda_ is not None and not (np.ndim(lambda_) == 0 and lambda_ == -1):
+        lam = np.ascontiguousarray(np.atleast_1d(lambda_), dtype=np.float64)
+        if len(lam) == 1 and lam[0] == -1:
+            lam = None
+        elif len(lam) != int(B_vec.sum()) + 1:
+            raise ValueError("lambda must hold B+1 values")
+    return B_vec, K, sigma, theta, lam
 
 
 class harmony:
@@ -89,7 +133,15 @@ class harmony:
               block_size, B_vec, batch_proportion_cutoff, verbose=False):
         """harmony::setup (harmony.h:25-30).  ``Z``: [N, d] C-order (== the d x N column-major matrix
         of the reference) or [d, N] F-order; ``Phi``: the row-index slot of the B x N design matrix,
-        int array [N, C]; ``lambda_``: B+1 values or None / -1 for automatic estimation."""
+        int array [N, C]; ``lambda_``: B+1 values or None / -1 for automatic estimation.
+
+        ``Z`` may also be a CUDA tensor (float32 / float64, [N, d] or [d, N], any strides) on this object's device;
+        ``Phi`` is then a numpy array or a CUDA integer tensor.  Both are read on the current CUDA stream and nothing
+        is copied through the host; the object ends in the state numpy input with the same values gives."""
+        torch = torch_of(Z)
+        if torch is not None and Z.is_cuda:
+            return self._setup_device(torch, Z, Phi, sigma, theta, lambda_, alpha, max_iter_kmeans, epsilon_kmeans,
+                                      epsilon_harmony, K, block_size, B_vec, batch_proportion_cutoff, verbose)
         Z = np.asarray(Z)
         phi_i = np.ascontiguousarray(Phi, dtype=np.int32)
         if phi_i.ndim == 1:
@@ -102,24 +154,67 @@ class harmony:
         Z = np.ascontiguousarray(Z, dtype=np.float64)
         if Z.shape[0] != n:
             raise ValueError("number of cells in Z and Phi differ")
-        B_vec = np.ascontiguousarray(np.atleast_1d(B_vec), dtype=np.int32)
-        K = int(K)
-        sigma = np.ascontiguousarray(np.broadcast_to(np.asarray(sigma, dtype=np.float64), (K,)))
-        theta = np.ascontiguousarray(theta, dtype=np.float64)
-        if len(theta) != int(B_vec.sum()):
-            raise ValueError("theta must hold one value per covariate level")
-        lam = None
-        if lambda_ is not None and not (np.ndim(lambda_) == 0 and lambda_ == -1):
-            lam = np.ascontiguousarray(np.atleast_1d(lambda_), dtype=np.float64)
-            if len(lam) == 1 and lam[0] == -1:
-                lam = None
-            elif len(lam) != int(B_vec.sum()) + 1:
-                raise ValueError("lambda must hold B+1 values")
+        B_vec, K, sigma, theta, lam = _setup_params(sigma, theta, lambda_, K, B_vec)
         self._check(self._L.hb_setup(self._h, _ptr(Z), Z.shape[1], n, _ptr(phi_i), _ptr(B_vec), len(B_vec),
                                      _ptr(sigma), _ptr(theta), None if lam is None else _ptr(lam), float(alpha),
                                      int(max_iter_kmeans), float(epsilon_kmeans), float(epsilon_harmony), K,
                                      float(block_size), float(batch_proportion_cutoff), int(bool(verbose))))
 
+    def _setup_device(self, torch, Z, Phi, sigma, theta, lambda_, alpha, max_iter_kmeans, epsilon_kmeans,
+                      epsilon_harmony, K, block_size, B_vec, batch_proportion_cutoff, verbose):
+        dev = torch.device("cuda", self._scalar("device"))
+        if Z.device != dev:
+            raise ValueError(f"Z is on {Z.device}, this harmony object on {dev}")
+        if torch_of(Phi) is not None:
+            if Phi.is_cuda and Phi.device != dev:
+                raise ValueError(f"Phi is on {Phi.device}, this harmony object on {dev}")
+            if Phi.dtype.is_floating_point or Phi.dtype.is_complex or Phi.dtype == torch.bool:
+                raise TypeError(f"Phi must hold integer level rows, not {Phi.dtype}")
+            phi = Phi.to(device=dev, dtype=torch.int32)
+        else:
+            phi = torch.from_numpy(np.ascontiguousarray(Phi, dtype=np.int32)).to(dev)
+        if phi.dim() == 1:
+            phi = phi.reshape(-1, 1)
+        phi = phi.contiguous()
+        n = phi.shape[0]
+        code, cell_stride, pc_stride, d = tensor_abi_args(Z, n)
+        B_vec, K, sigma, theta, lam = _setup_params(sigma, theta, lambda_, K, B_vec)
+        self._check(self._L.hb_setup_device(
+            self._h, Z.data_ptr(), code, cell_stride, pc_stride, d, n, phi.data_ptr(), _ptr(B_vec), len(B_vec),
+            _ptr(sigma), _ptr(theta), None if lam is None else _ptr(lam), float(alpha), int(max_iter_kmeans),
+            float(epsilon_kmeans), float(epsilon_harmony), K, float(block_size), float(batch_proportion_cutoff),
+            int(bool(verbose)), torch.cuda.current_stream(dev).cuda_stream))
+
+    def to_torch(self, field="Z_corr", dtype=None, out=None):
+        """A per-cell field as a CUDA tensor on this object's device, cells as rows: ``"Z_corr"`` / ``"Z_orig"``
+        [N_local, d], ``"R"`` [N_local, K]; float32 unless ``dtype`` (float32 / float64) says otherwise.  ``out``: a
+        preallocated tensor of that shape whose rows may be strided (e.g. a column slice of a wider tensor).  Ordered on
+        the current CUDA stream without a host synchronisation; values are those of getZcorr() / getZorig() / R."""
+        import torch
+        cols = {"Z_corr": "d", "Z_orig": "d", "R": "K"}
+        if field not in cols:
+            raise ValueError(f"field must be one of {sorted(cols)}, not {field!r}")
+        dev = torch.device("cuda", self._scalar("device"))
+        shape = (self._scalar("N_local"), self._scalar(cols[field]))
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32 if dtype is None else dtype, device=dev)
+        elif torch_of(out) is None or tuple(out.shape) != shape or out.device != dev or \
+                (out.stride(1) != 1 and shape[1] > 1) or (dtype is not None and out.dtype != dtype):
+            raise ValueError(f"out must be a {dtype or 'float'} tensor of shape {shape} on {dev} with unit column stride")
+        codes = {torch.float32: HB_F32, torch.float64: HB_F64}
+        if out.dtype not in codes:
+            raise TypeError(f"to_torch writes float32 or float64, not {out.dtype}")
+        ld = out.stride(0) if shape[0] > 1 else shape[1]
+        self._check(self._L.hb_get_field_device(self._h, FIELD[field], out.data_ptr(), codes[out.dtype], ld,
+                                                torch.cuda.current_stream(dev).cuda_stream))
+        return out
+
+    def debug_sort_perm(self):
+        """Test hook: the tuple-sort permutation (position -> local cell)."""
+        out = np.empty(self._scalar("N_local"), dtype=np.int32)
+        if self._L.hb_debug_sort_perm(self._h, _ptr(out)) != 0:
+            raise HarmonyError("hb_debug_sort_perm failed (setup has not run?)")
+        return out
     def set_seed(self, seed):
         self._check(self._L.hb_set_seed(self._h, int(seed) & 0xFFFFFFFFFFFFFFFF))
 

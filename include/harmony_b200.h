@@ -16,6 +16,7 @@
  *     phi_i[n*C + c] is the (global, 0-based) row of the c-th non-zero of column n.
  *   - all buffers are caller-owned host memory; inputs are copied during the call
  *     (like harmony::setup, harmony.cpp:41,44), outputs are written into caller-allocated arrays.
+ *     The *_device entry points take / fill caller-owned DEVICE memory instead (cells as rows, any strides).
  *   - a handle must be driven from one host thread at a time (the reference is single-threaded).
  */
 #ifndef HARMONY_B200_H
@@ -63,6 +64,23 @@ int hb_setup(hb_handle* h, const double* Z, int d, int64_t N, const int32_t* phi
              const double* sigma, const double* theta, const double* lambda, double alpha, int max_iter_kmeans,
              double epsilon_kmeans, double epsilon_harmony, int K, double block_size,
              double batch_proportion_cutoff, int verbose);
+
+/* Element types of caller device memory (hb_setup_device, hb_get_field_device). */
+enum hb_dtype { HB_F32 = 0, HB_F64 = 1 };
+
+/* harmony::setup with the per-cell inputs in device memory of the handle's device.
+ * Z: N cells x d PCs, element (n, c) at Z[n*z_cell_stride + c*z_pc_stride] (elements, not bytes), HB_F32/HB_F64.
+ *    Covers a contiguous [N, d] tensor, its [d, N] transpose view and column slices, without a copy.
+ * phi_i: device int32, N x C row-major, same meaning as hb_setup's phi_i (global level row).
+ * B_vec, sigma, theta, lambda and the scalars: host memory, exactly as in hb_setup.
+ * stream: the caller's cudaStream_t on which Z and phi_i are ready (NULL = legacy default stream).
+ * The inputs are fully consumed before the call returns, so the caller may free them afterwards.
+ * The handle ends in the state hb_setup leaves it in for the same values (Z converted to float as hb_setup does). */
+int hb_setup_device(hb_handle* h, const void* Z, int z_dtype, int64_t z_cell_stride, int64_t z_pc_stride, int d,
+                    int64_t N, const int32_t* phi_i, const int32_t* B_vec, int C, const double* sigma,
+                    const double* theta, const double* lambda, double alpha, int max_iter_kmeans,
+                    double epsilon_kmeans, double epsilon_harmony, int K, double block_size,
+                    double batch_proportion_cutoff, int verbose, void* stream);
 
 /* Seed of the native generators (k-means initialisation, per-round update orders).  The reference
  * draws both from R's RNG (utils.cpp:10-64, harmony.cpp:272-273); the shim may instead inject them. */
@@ -113,10 +131,15 @@ int hb_get_field(hb_handle* h, int field, double* out);
 /* Writable fields (the Rcpp module's .field() members are read-write): HB_Y, HB_R, HB_O, HB_E,
  * HB_THETA, HB_SIGMA, HB_LAMBDA_VEC, HB_Z_CORR. */
 int hb_set_field(hb_handle* h, int field, const double* in);
+/* Per-cell fields (HB_Z_CORR, HB_Z_ORIG, HB_R) un-sorted into caller device memory: N_local rows of d (or K)
+ * values, row stride ld elements, HB_F32 or HB_F64.  Ordered on `stream`: the library waits for the stream
+ * before writing and makes the stream wait for the write, so there is no host synchronisation. */
+int hb_get_field_device(hb_handle* h, int field, void* out, int dtype, int64_t ld, void* stream);
 
 enum hb_scalar { HB_N = 0, HB_B = 1, HB_K = 2, HB_D = 3, HB_C = 4, HB_ALPHA = 5, HB_MAX_ITER_KMEANS = 6,
                  HB_BLOCK_SIZE = 7, HB_EPSILON_KMEANS = 8, HB_EPSILON_HARMONY = 9, HB_N_LOCAL = 10,
-                 HB_LAMBDA_ESTIMATION = 11, HB_WINDOW_SIZE = 12, HB_LEGACY_CENTROID_STEP = 13, HB_KERNEL_SET = 14 };
+                 HB_LAMBDA_ESTIMATION = 11, HB_WINDOW_SIZE = 12, HB_LEGACY_CENTROID_STEP = 13, HB_KERNEL_SET = 14,
+                 HB_DEVICE = 15 /* CUDA device of the handle (read-only) */ };
 /* HB_KERNEL_SET (test hook, default 0, read by the next hb_setup): the library picks its kernels from the problem's
  * shape alone; these bits force the kernels that serve shapes outside the default ones' limits onto ANY shape so that
  * the parity suite can hold them to the same bar (tests/test_gpu_parity.py::test_fallback_kernels_match_oracle). */
@@ -159,6 +182,8 @@ uint64_t hb_debug_permute(uint64_t i, uint64_t n, uint64_t key, int inverse);
 /* Test hook (host only): the host worker pool of the download path (hb_get_field) widens n floats to
  * doubles; `threads` sizes the pool on first use (<= 0: HB_HOST_THREADS or the core count).  Returns the pool size. */
 int hb_debug_widen(double* out, const float* in, int64_t n, int threads);
+/* Test hook: the tuple-sort permutation (position -> local cell), N_local int32 values. */
+int hb_debug_sort_perm(const hb_handle* h, int32_t* out);
 /* Test hooks of the native kmeans_centers (hb_init_cluster(h, NULL); utils.cpp:10-64): the keyed-hash uniform that
  * stands in for arma::randu at (centroid i, global cell g) — i = K addresses the K start-cell draws — and the global
  * cells initialize_centroids chose (returns their number, 0 if the native initialisation has not run). */
